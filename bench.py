@@ -7,7 +7,12 @@ DEM (1.07 Gcells; 4 GiB, far larger than the 126 MB L2, so no cache flush is nee
 steps).  `value` = cells / device time with the DEM resident in HBM; `e2e` = the same two calls
 through the host-pointer C ABI (pinned host buffers, H2D/D2H inside the timed region).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--size 32768] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--size 32768] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step computed, the filled DEM (DIR/filled.npy, float32) and its D8
+accumulation (DIR/fa_d8.npy, float64): whole rasters up to DUMP_CELLS cells, above that the same seeded sample of
+DUMP_CELLS cells in every run of a size, so that two builds (or, at the same raster size, the GPU path and
+--impl reference) can be compared output for output.
 
 After the timed loop the result of the last step is VERIFIED on the device (fixed-point equation of the fill,
 pinned border, conservation of the D8 accumulation) and position-weighted 64-bit checksums of the filled raster and
@@ -102,9 +107,10 @@ class ClockSampler:
 
 
 # ---------------------------------------------------------------------------------------------
-def cpu_reference_run(n: int, steps: int, warmup: int, budget_s: float = 1e9):
+def cpu_reference_run(n: int, steps: int, warmup: int, budget_s: float = 1e9, dump_dir=None):
     """Times the CPU implementation (reference if compiled, else port) on the n x n benchmark raster (the device
-    generator's bit-identical CPU restatement).  Stops early (after >= 1 timed step) when `budget_s` is spent."""
+    generator's bit-identical CPU restatement).  Stops early (after >= 1 timed step) when `budget_s` is spent.
+    dump_dir: write the last step's outputs there as --dump-outputs does for the GPU path."""
     import oracle
     O = oracle.best()
     kind = "reference" if O.kind == "reference" else "port"
@@ -115,16 +121,21 @@ def cpu_reference_run(n: int, steps: int, warmup: int, budget_s: float = 1e9):
     times = []
     t_start = time.perf_counter()
     for i in range(warmup + steps):
+        f = a = None
         t = time.perf_counter()
         f = O.fill_depressions(dem)
         t1 = time.perf_counter()
         a = O.fa_d8(f, ND)
         t2 = time.perf_counter()
-        del a, f
         if i >= warmup:
             times.append((t2 - t, t1 - t, t2 - t1))
         if times and time.perf_counter() - t_start > budget_s:
             break
+    if dump_dir:
+        idx = dump_indices(n, n)
+        save_dump(dump_dir, "filled", f.reshape(-1)[idx], n, n)
+        save_dump(dump_dir, "fa_d8", a.reshape(-1)[idx], n, n)
+    del a, f
     tot = sum(t[0] for t in times) / len(times)
     return {
         "value": n * n / tot / 1e6, "unit": UNIT, "cores": cores, "kind": kind,
@@ -159,7 +170,8 @@ def run_reference(args):
     if args.ref_size:
         n = args.ref_size
     # one full-size step costs minutes of serial CPU: cap the number of steps by wall time, not the raster
-    cb = cpu_reference_run(n, max(1, args.steps), 0 if n >= 8192 else max(0, min(args.warmup, 1)), budget_s=args.ref_budget_s)
+    cb = cpu_reference_run(n, max(1, args.steps), 0 if n >= 8192 else max(0, min(args.warmup, 1)), budget_s=args.ref_budget_s,
+                           dump_dir=args.dump_outputs)
     line = {
         "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": cb["seconds_per_run"] * 1e3,
@@ -190,6 +202,44 @@ def _checksum(t, row0, width):
         idx = (torch.arange(blk.numel(), device=t.device, dtype=torch.int64) + (row0 + y) * width) % 1000003 + 1
         tot += (bits.reshape(-1) * idx).sum()
     return tot
+
+
+DUMP_CELLS = 1 << 22  # at most 16 MiB of elevations + 32 MiB of accumulation
+
+
+def dump_indices(N, W):
+    """Flat cell indices --dump-outputs writes: all N * W when they are at most DUMP_CELLS, else the sorted, seeded
+    sample np.unique(default_rng(SEED).integers(0, N * W, DUMP_CELLS)), the same in every run of a size."""
+    import numpy as np
+    cells = N * W
+    return np.arange(cells) if cells <= DUMP_CELLS else np.unique(np.random.default_rng(SEED).integers(0, cells, DUMP_CELLS))
+
+
+def save_dump(out_dir, name, values, N, W):
+    """values (at dump_indices(N, W)) -> out_dir/<name>.npy, as the N x W raster when it is whole."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), values.reshape(N, W) if N * W <= DUMP_CELLS else values)
+
+
+def dump_outputs(out_dir, filled, acc, r0, r1, gt, N, W, world, rank):
+    """Writes filled.npy and fa_d8.npy of the GPU path (see --dump-outputs).  filled / acc are local rasters (gt ghost
+    rows + rows r0 .. r1 of the raster + ghost rows); ranks add their cells."""
+    import numpy as np
+    import torch
+    import torch.distributed as dist
+    idx = dump_indices(N, W)
+    rows = idx // W
+    mine = np.nonzero((rows >= r0) & (rows < r1))[0]
+    src = torch.from_numpy((rows[mine] - r0 + gt) * W + idx[mine] % W).cuda()
+    dst = torch.from_numpy(mine).cuda()
+    for name, t in (("filled", filled), ("fa_d8", acc)):
+        v = torch.zeros(len(idx), dtype=t.dtype, device="cuda")
+        v[dst] = t.reshape(-1)[src]
+        if world > 1:
+            dist.all_reduce(v)
+        if rank == 0:
+            save_dump(out_dir, name, v.cpu().numpy(), N, W)
 
 
 def verify_band(z_loc, w_loc, acc_loc, gt, gb, r0, r1, H, W):
@@ -339,6 +389,9 @@ def run_b200(args):
     ms_per_step = dev_ms / args.steps
     cells = float(N) * float(N)
     value = cells / (ms_per_step * 1e-3) / 1e6
+
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last["filled"], last["acc"], r0, r1, gt, N, W, world, rank)
 
     # ---- verification of what was just timed (the last step's outputs), at every N ----
     verification = None
@@ -668,7 +721,11 @@ def main():
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--traffic", type=float, default=None,
                     help="dram bytes per sweep launch from the committed ncu capture (default: profiles/traffic.json)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's filled DEM and D8 accumulation as DIR/<name>.npy (see the module doc)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.dominant_launch = None
     try:
         tj = json.load(open(os.path.join(ROOT, "profiles", "traffic.json")))

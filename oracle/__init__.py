@@ -43,6 +43,14 @@ def build(force: bool = False) -> None:
                               stderr=subprocess.DEVNULL)
 
 
+def build_bindings() -> None:
+    """Compile the reference's C++ drop-in check and its Python module over librichdem_b200.so into
+    build/reference_bindings/ (oracle/Makefile `bindings`; nothing happens where the reference's sources are absent).
+    Compiler errors reach stderr."""
+    import sys
+    subprocess.check_call(["make", "-C", _HERE, "bindings", f"PYTHON={sys.executable}"], stdout=subprocess.DEVNULL)
+
+
 def have_ref() -> bool:
     return os.path.exists(_REF_PATH)
 
@@ -319,6 +327,16 @@ def ref() -> _Backend:
 def best() -> _Backend:
     """Reference when it was built here, else the port."""
     return ref() if have_ref() else port()
+
+
+def digest(a) -> str:
+    """SHA-256 of an array's dtype, shape and C-order bytes: how tests/golden/reference_digests.json pins whole outputs
+    of the reference that would be too large to store."""
+    import hashlib
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(f"{a.dtype.str} {a.shape}".encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
 
 
 def device_fbm(h: int, w: int, seed: int = 42, octaves: int = 12, quantum: float = 0.0, y0: int = 0) -> np.ndarray:

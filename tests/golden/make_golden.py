@@ -108,6 +108,9 @@ def main():
     metrics()
     flowdirs_flats()
     terrain_attributes()
+    reference_digests()
+    epsilon_fill()
+    native_cache()
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))
 
@@ -161,6 +164,95 @@ def terrain_attributes():
     np.savez_compressed(f"{OUT}/terrain_attributes_ref.npz", **out)
 
 
+ND = -9999.0
+PORT_CASES = [(7, (97, 133), None, False), (8, (160, 120), 0.5, True), (9, (300, 300), 4.0, False)]
+D4_CASES = [(7, (97, 133), None), (8, (160, 120), 0.5), (9, (300, 300), 4.0)]
+TA_LIVE_CASES = [(1.0, (1.0, 1.0), -9999.0), (0.3048, (10.0, 10.0), -1.0), (3.0, (5.0, 7.5), -9999.0)]
+
+
+def reference_digests():
+    """9. whole outputs of the unmodified reference on the seeded synthetic DEMs of tests/test_oracle.py and on the 8192^2
+    benchmark raster of tests/test_gpu_parity.py, as oracle.digest() values (the arrays themselves are megabytes): the
+    inputs are regenerated at test time from their seeds and the C port / the GPU must reproduce every digest."""
+    import json
+    R = oracle.ref()
+    dg = oracle.digest
+    out = {}
+    for seed, shape, q, patch in PORT_CASES:
+        dem = oracle.fbm_terrain(*shape, seed=seed, quantum=q)
+        if patch:
+            dem[20:50, 30:70] = ND
+            dem[:9, :13] = ND
+        f = R.fill_depressions(dem)
+        m, l = R.flat_mask(f, ND)
+        r = R.resolve_flats(f, ND)
+        d = R.d8_flow_directions(r, ND)
+        wts = np.random.default_rng(seed).random(shape)
+        out[f"port_s{seed}"] = {
+            "dem": dg(dem), **{f"fill_{v}": dg(R.fill_depressions(dem, v)) for v in (None, "fill_zhou", "fill_barnes", "fill_original")},
+            "find_flats": dg(R.find_flats(f, ND)), "flat_mask": dg(m), "flat_labeled": dg(l != 0), "resolved": dg(r),
+            "dirs": dg(d), "d8_flow_accum": dg(R.d8_flow_accum(d)), "fm_d8": dg(R.fm_d8(r, ND)), "fm_dinf": dg(R.fm_dinf(r, ND)),
+            "fa_d8": dg(R.fa_d8(r, ND)), "fa_dinf": dg(R.fa_dinf(r, ND)), "fa_dinf_weighted": dg(R.fa_dinf(r, ND, wts))}
+    dem = oracle.fbm_terrain(140, 190, seed=21, quantum=0.5)
+    dem[20:40, 30:70] = ND
+    wts = np.random.default_rng(3).random(dem.shape)
+    out["metrics_s21"] = {"dem": dg(dem)}
+    for m, e in METRIC_CASES:
+        out["metrics_s21"][f"{m}_{e}"] = {"fm": dg(R.fm_method(dem, ND, m, e)), "fa": dg(R.fa_method(dem, ND, m, e)),
+                                          "fa_weighted": dg(R.fa_method(dem, ND, m, e, wts))}
+    for seed, shape, q in D4_CASES:
+        dem = oracle.fbm_terrain(*shape, seed=seed, quantum=q)
+        dem[20:40, 30:60] = ND
+        out[f"fill_d4_s{seed}"] = {"dem": dg(dem), "fill_d4": dg(R.fill_depressions(dem, "fill_d4"))}
+    dem = R.fill_depressions(oracle.fbm_terrain(180, 150, seed=33, quantum=1.0))
+    dem[60:80, 40:70] = ND
+    dirs, m, l = R.d8_flow_directions_flats(dem, ND)
+    out["flowdirs_flats_s33"] = {"dem": dg(dem), "dirs": dg(dirs), "mask": dg(m), "labeled": dg(l != 0)}
+    dem = oracle.fbm_terrain(150, 211, seed=23, quantum=0.5)
+    dem[20:40, 30:70] = ND
+    dem[0, :9] = ND
+    out["terrain_s23"] = {"dem": dg(dem)}
+    for attrib in R.TA_IDS:
+        for zs, cell, nd_out in TA_LIVE_CASES:
+            out["terrain_s23"][f"{attrib}__{zs}"] = dg(R.terrain_attribute(dem, attrib, ND, zs, cell, nd_out))
+    dem = oracle.device_fbm(8192, 8192, seed=42)
+    f = R.fill_depressions(dem)
+    out["bench_8192"] = {"dem": dg(dem), "filled": dg(f), "fa_d8": dg(R.fa_d8(f, ND))}
+    with open(f"{OUT}/reference_digests.json", "w") as fh:
+        json.dump(out, fh, indent=1, sort_keys=True)
+        fh.write("\n")
+
+
+def epsilon_fill():
+    """10. PriorityFloodEpsilon_Barnes2014 (depressions/Barnes2014.hpp:336-420) of the unmodified reference on three seeded
+    60 x 80 synthetic DEMs, whole (tests/test_oracle.py::test_epsilon_fill_depends_on_the_queue_order)."""
+    import ctypes as C
+    R = oracle.ref()
+    f = R.lib.ref_priority_flood_epsilon_f32
+    f.argtypes = [np.ctypeslib.ndpointer(np.float32, flags="C_CONTIGUOUS"), C.c_int, C.c_int, C.c_float]
+    f.restype = None
+    out = {}
+    for seed in (2, 5, 7):
+        z = oracle.fbm_terrain(60, 80, seed=seed, quantum=0.5)
+        ref = z.copy()
+        f(ref, 80, 60, ND)
+        out[f"s{seed}__dem"], out[f"s{seed}__epsilon_filled"] = z, ref
+    np.savez_compressed(f"{OUT}/epsilon_fill_ref.npz", **out)
+
+
+def native_cache():
+    """11. a file in richdem::Array2D's native cache format (common/Array2D.hpp:209-281) written by the unmodified
+    reference; the reference reads it back bit for bit, metadata included."""
+    R = oracle.ref()
+    dem = oracle.fbm_terrain(37, 53, seed=3)
+    dem[5:9, 7:20] = ND
+    gt = [100.0, 30.0, 0.0, 2000.0, 0.0, -20.0]
+    path = f"{OUT}/native_cache_ref.rd"
+    R.save_native(path, dem, ND, gt, "EPSG:26915")
+    data, nd, gt2, proj = R.load_native(path)
+    assert np.array_equal(data.view(np.uint32), dem.view(np.uint32)) and nd == ND and list(gt2) == gt and proj == "EPSG:26915"
+
+
 if __name__ == "__main__":
     if "--metrics-only" in sys.argv:
         metrics()
@@ -168,5 +260,9 @@ if __name__ == "__main__":
         flowdirs_flats()
     elif "--terrain-attributes-only" in sys.argv:
         terrain_attributes()
+    elif "--reference-digests-only" in sys.argv:
+        reference_digests()
+        epsilon_fill()
+        native_cache()
     else:
         main()

@@ -6,7 +6,7 @@
 // through -I<reference>/wrappers/pyrichdem/src at compile time; nothing of it is copied into this repository) follows.
 // The resulting module serves richdem/__init__.py unchanged: FillDepressions, ResolveFlats, FlowAccumulation and
 // FlowProportions on float32 rasters run on the GPU, every other dtype / method keeps the reference's CPU templates.
-// Built by __graft_entry__.build() into tests/_bin/pyrichdem/ (git-ignored; travels to the GPU box like oracle/_ref).
+// Built by oracle/Makefile (`bindings`) into build/reference_bindings/pyrichdem/ (git-ignored).
 #include <richdem_b200.hpp>
 
 #include <pywrapper.cpp>

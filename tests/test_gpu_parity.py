@@ -3,6 +3,9 @@ librichdem_b200.so (via the Python mirror of the reference API) and is compared 
 checker on the same inputs: bit-exact for filled elevations, flat masks, resolved elevations,
 direction grids, FM_D8 proportions and unit-weight D8 accumulation; <= 1 float ulp for D-infinity
 proportions; 1e-9 relative (north_star allows 1e-5) for weighted / D-infinity accumulation."""
+import json
+import os
+
 import numpy as np
 import pytest
 
@@ -246,9 +249,9 @@ def test_cxx_dropin_matches_reference_cpu_templates():
     the reference's own CPU templates instantiated for double (in-process oracle inside the binary)."""
     import os
     import subprocess
-    exe = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "_bin", "cxx_dropin_check")
+    exe = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "build", "reference_bindings", "cxx_dropin_check")
     if not os.path.exists(exe):
-        pytest.skip("tests/_bin/cxx_dropin_check not built (reference headers absent at build time)")
+        pytest.skip("build/reference_bindings/cxx_dropin_check not built (reference headers absent at build time)")
     out = subprocess.run([exe], capture_output=True, text=True)
     assert out.returncode == 0, out.stdout[-3000:]
     assert "thrown=0 mismatches=0 dim_mismatch_throws=1" in out.stdout, out.stdout[-3000:]
@@ -387,16 +390,17 @@ def test_device_terrain_generator_equals_its_cpu_restatement():
         assert np.array_equal(d.cpu().numpy().view(np.uint32), oracle.device_fbm(h, w, seed=seed, quantum=q, y0=y0).view(np.uint32))
 
 
-@pytest.mark.skipif(not oracle.have_ref(), reason="needs the compiled reference (about 20 s of CPU for 8192^2)")
-def test_fill_and_d8_accumulation_vs_reference_at_8192(checker):
-    """The benchmark workload at 8192^2 (67 Mcells) against the compiled reference: fill bit-exact, FA_D8 bit-exact."""
+def test_fill_and_d8_accumulation_vs_reference_at_8192():
+    """The benchmark workload at 8192^2 (67 Mcells) against the reference: fill bit-exact, FA_D8 bit-exact (digests of the
+    reference's whole outputs, tests/golden/make_golden.py::reference_digests)."""
     N = 8192
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_digests.json")) as f:
+        D = json.load(f)["bench_8192"]
     dem = oracle.device_fbm(N, N, seed=42)
-    f_ref = checker.fill_depressions(dem)
+    assert oracle.digest(dem) == D["dem"], "benchmark raster drifted"
     filled = np.asarray(rd.FillDepressions(R(dem)))
-    assert np.array_equal(filled, f_ref)
-    a_ref = checker.fa_d8(f_ref, ND)
-    assert np.array_equal(np.asarray(rd.FlowAccumulation(R(filled), "D8")), a_ref)
+    assert oracle.digest(filled) == D["filled"]
+    assert oracle.digest(np.asarray(rd.FlowAccumulation(R(filled), "D8"))) == D["fa_d8"]
 
 
 # ---- FillDepressions<Topology::D4> ---------------------------------------------------------------------------

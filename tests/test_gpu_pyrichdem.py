@@ -1,8 +1,8 @@
 """SURVEY 8b-2: the reference's OWN Python package on the B200 path.
 
-tests/_bin/pyrichdem/ (built by __graft_entry__.build() where /root/reference exists; git-ignored, travels to the GPU
-box) holds
-  * `_richdem.*.so`  -- the reference's pybind11 binding source (wrappers/pyrichdem/src/pywrapper.cpp), unmodified,
+build/reference_bindings/pyrichdem/ (built by oracle/Makefile where the reference's sources are available; git-ignored)
+holds
+  * `_richdem.so`    -- the reference's pybind11 binding source (wrappers/pyrichdem/src/pywrapper.cpp), unmodified,
                         compiled with include/richdem_b200.hpp in front of it (tests/pyrichdem_module.cpp), so that
                         rdFillDepressionsD8 / rdResolveFlatsEpsilon / FA_* / FM_* / FlowAccumulation on float32 rasters
                         are the explicit specialisations that call librichdem_b200.so;
@@ -18,7 +18,7 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
-PKG = os.path.join(HERE, "_bin", "pyrichdem")
+PKG = os.path.join(os.path.dirname(HERE), "build", "reference_bindings", "pyrichdem")
 ND = -9999.0
 
 
@@ -26,7 +26,7 @@ ND = -9999.0
 def rdref():
     if not os.path.exists(os.path.join(PKG, "richdem", "__init__.pyc")) or not any(
             f.startswith("_richdem") for f in os.listdir(PKG)):
-        pytest.skip("tests/_bin/pyrichdem not built (reference tree absent at build time)")
+        pytest.skip("build/reference_bindings/pyrichdem not built (reference tree absent at build time)")
     sys.path.insert(0, PKG)
     try:
         import richdem  # the reference package, unmodified

@@ -1,14 +1,39 @@
 """Pins the CPU oracle (oracle/oracle.c) before anything trusts it:
   * against the reference's own known-answer fixtures (re-encoded in tests/golden/),
   * against stored outputs of the unmodified reference on real + synthetic terrain,
-  * live against oracle/_ref (the compiled reference) when it is available.
+  * against digests of whole outputs of the unmodified reference on seeded synthetic terrain
+    (tests/golden/reference_digests.json, written by tests/golden/make_golden.py from oracle/_ref).
 No GPU involved."""
+import json
+import os
+
 import numpy as np
 import pytest
 
 import oracle
 
 ND = -9999.0
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+with open(os.path.join(GOLDEN, "reference_digests.json")) as _f:
+    REF = json.load(_f)
+
+
+def assert_digests(expected, **arrays):
+    """Each array's oracle.digest() equals the stored digest of the reference's output of the same name.  Only digests
+    are stored, so a failure names the outputs and what they hold; tests/golden/make_golden.py::reference_digests shows
+    the reference call that produced each one, for a cell-by-cell comparison where the reference is at hand."""
+    bad = []
+    for k, a in arrays.items():
+        got = oracle.digest(a)
+        if got != expected[k]:
+            a = np.asarray(a)
+            what = f"{a.dtype} {a.shape}" + (f", min {a.min()}, max {a.max()}" if a.size else "")
+            if a.dtype == bool:
+                what += f", {np.count_nonzero(a)} set"
+            elif a.dtype.kind == "f":
+                what += f", {np.count_nonzero(~np.isfinite(a))} non-finite"
+            bad.append(f"{k}: {what}; digest {got[:16]} instead of the reference's {expected[k][:16]}")
+    assert not bad, "differs from the reference:\n  " + "\n  ".join(bad)
 
 
 def test_fill_known_answer(port, golden):
@@ -71,32 +96,27 @@ def test_synthetic_against_reference_outputs(port, golden):
         assert np.array_equal(port.fa_dinf(r, ND), g[f"{k}__fa_dinf"])
 
 
-@pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref not built (no reference tree)")
 @pytest.mark.parametrize("seed,shape,q,nodata_patch", [(7, (97, 133), None, False), (8, (160, 120), 0.5, True),
                                                        (9, (300, 300), 4.0, False)])
 def test_port_matches_compiled_reference_live(port, seed, shape, q, nodata_patch):
-    R = oracle.ref()
+    """The whole pipeline, bit for bit, against the reference's outputs (tests/golden/make_golden.py::reference_digests;
+    the fill against all four of the reference's Priority-Flood variants)."""
+    D = REF[f"port_s{seed}"]
     dem = oracle.fbm_terrain(*shape, seed=seed, quantum=q)
     if nodata_patch:
         dem[20:50, 30:70] = ND
         dem[:9, :13] = ND
+    assert_digests(D, dem=dem)
     f = port.fill_depressions(dem)
-    for variant in (None, "fill_zhou", "fill_barnes", "fill_original"):
-        assert np.array_equal(f, R.fill_depressions(dem, variant))
-    assert np.array_equal(port.find_flats(f, ND), R.find_flats(f, ND))
-    (m1, l1), (m2, l2) = port.flat_mask(f, ND), R.flat_mask(f, ND)
-    assert np.array_equal(m1, m2) and np.array_equal(l1 != 0, l2 != 0)
+    assert_digests(D, **{f"fill_{v}": f for v in (None, "fill_zhou", "fill_barnes", "fill_original")})
+    m, l = port.flat_mask(f, ND)
+    assert_digests(D, find_flats=port.find_flats(f, ND), flat_mask=m, flat_labeled=l != 0)
     r = port.resolve_flats(f, ND)
-    assert np.array_equal(r, R.resolve_flats(f, ND))
     d = port.d8_flow_directions(r, ND)
-    assert np.array_equal(d, R.d8_flow_directions(r, ND))
-    assert np.array_equal(port.d8_flow_accum(d), R.d8_flow_accum(d))
-    assert np.array_equal(port.fm_d8(r, ND), R.fm_d8(r, ND))
-    assert np.array_equal(port.fm_dinf(r, ND), R.fm_dinf(r, ND))
-    assert np.array_equal(port.fa_d8(r, ND), R.fa_d8(r, ND))
-    assert np.array_equal(port.fa_dinf(r, ND), R.fa_dinf(r, ND))
     wts = np.random.default_rng(seed).random(shape)
-    assert np.array_equal(port.fa_dinf(r, ND, wts), R.fa_dinf(r, ND, wts))
+    assert_digests(D, resolved=r, dirs=d, d8_flow_accum=port.d8_flow_accum(d), fm_d8=port.fm_d8(r, ND),
+                   fm_dinf=port.fm_dinf(r, ND), fa_d8=port.fa_d8(r, ND), fa_dinf=port.fa_dinf(r, ND),
+                   fa_dinf_weighted=port.fa_dinf(r, ND, wts))
 
 
 def test_fill_is_min_over_paths_of_max(port):
@@ -139,26 +159,23 @@ def test_remaining_flow_metrics_against_reference_outputs(port, golden):
             assert np.array_equal(port.fa_method(dem, ND, m, e)[::3, ::3], g[k + "__fa"]), k
 
 
-@pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref not built (no reference tree)")
 @pytest.mark.parametrize("method,exponent", METRIC_CASES)
 def test_remaining_flow_metrics_port_matches_compiled_reference_live(port, method, exponent):
-    R = oracle.ref()
     dem = oracle.fbm_terrain(140, 190, seed=21, quantum=0.5)
     dem[20:40, 30:70] = ND
-    assert np.array_equal(port.fm_method(dem, ND, method, exponent), R.fm_method(dem, ND, method, exponent))
-    assert np.array_equal(port.fa_method(dem, ND, method, exponent), R.fa_method(dem, ND, method, exponent))
+    assert_digests(REF["metrics_s21"], dem=dem)
     wts = np.random.default_rng(3).random(dem.shape)
-    assert np.array_equal(port.fa_method(dem, ND, method, exponent, wts), R.fa_method(dem, ND, method, exponent, wts))
+    assert_digests(REF["metrics_s21"][f"{method}_{exponent}"], fm=port.fm_method(dem, ND, method, exponent),
+                   fa=port.fa_method(dem, ND, method, exponent), fa_weighted=port.fa_method(dem, ND, method, exponent, wts))
 
 
-@pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref not built (no reference tree)")
 @pytest.mark.parametrize("seed,shape,q", [(7, (97, 133), None), (8, (160, 120), 0.5), (9, (300, 300), 4.0)])
 def test_d4_fill_port_matches_compiled_reference_live(port, seed, shape, q):
     """FillDepressions<Topology::D4> (depressions/depressions.hpp:16-17)."""
     dem = oracle.fbm_terrain(*shape, seed=seed, quantum=q)
     dem[20:40, 30:60] = ND
     d4 = port.fill_depressions(dem, "fill_d4")
-    assert np.array_equal(d4, oracle.ref().fill_depressions(dem, "fill_d4"))
+    assert_digests(REF[f"fill_d4_s{seed}"], dem=dem, fill_d4=d4)
     assert (d4 >= port.fill_depressions(dem)).all() and (d4 > port.fill_depressions(dem)).any(), "D4 fills at least as high as D8"
 
 
@@ -173,13 +190,11 @@ def test_direction_grid_flat_resolution_against_reference_outputs(port, golden):
         assert not ((dirs == 0) & inner & (l != 0)).any(), "every cell of a drainable flat received a direction"
 
 
-@pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref not built (no reference tree)")
 def test_direction_grid_flat_resolution_port_matches_compiled_reference_live(port):
     dem = port.fill_depressions(oracle.fbm_terrain(180, 150, seed=33, quantum=1.0))
     dem[60:80, 40:70] = ND
-    a = port.d8_flow_directions_flats(dem, ND)
-    b = oracle.ref().d8_flow_directions_flats(dem, ND)
-    assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]) and np.array_equal(a[2] != 0, b[2] != 0)
+    dirs, m, l = port.d8_flow_directions_flats(dem, ND)
+    assert_digests(REF["flowdirs_flats_s33"], dem=dem, dirs=dirs, mask=m, labeled=l != 0)
 
 
 # ---- SURVEY 8f-4: terrain attributes --------------------------------------------------------------------------------------
@@ -197,34 +212,28 @@ def test_terrain_attributes_against_reference_outputs(port, golden):
                 assert np.array_equal(got.view(np.uint32), g[f"{name}__{attrib}__{zs}"].view(np.uint32)), (name, attrib, zs)
 
 
-@pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref not built (no reference tree)")
 def test_terrain_attributes_port_matches_compiled_reference_live(port):
-    R = oracle.ref()
     dem = oracle.fbm_terrain(150, 211, seed=23, quantum=0.5)
     dem[20:40, 30:70] = ND
     dem[0, :9] = ND
+    assert_digests(REF["terrain_s23"], dem=dem)
     for attrib in port.TA_IDS:
         for zs, cell, nd_out in ((1.0, (1.0, 1.0), -9999.0), (0.3048, (10.0, 10.0), -1.0), (3.0, (5.0, 7.5), -9999.0)):
             a = port.terrain_attribute(dem, attrib, ND, zs, cell, nd_out)
-            b = R.terrain_attribute(dem, attrib, ND, zs, cell, nd_out)
-            assert np.array_equal(a.view(np.uint32), b.view(np.uint32)), (attrib, zs)
+            assert_digests(REF["terrain_s23"], **{f"{attrib}__{zs}": a})
             assert np.all(a[dem == ND] == nd_out)
 
 
 # ---- SURVEY 8f-3: why the epsilon fill is not on the B200 path -----------------------------------------------------------
-@pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref not built (no reference tree)")
-def test_epsilon_fill_depends_on_the_queue_order():
+def test_epsilon_fill_depends_on_the_queue_order(golden):
     """PriorityFloodEpsilon_Barnes2014 (depressions/Barnes2014.hpp:336-420) drains its FIFO "pit" queue before it looks at the
     priority queue again (:377-392), so a pit cell can be closed from a neighbour that is not its cheapest one: the result is
     NOT the order-free fixed point W = max(Z, min_n nextafter(W_n)) a parallel relaxation converges to -- it lies up to a few
     float ulps above it in a few cells.  A bit-exact GPU version would have to replay the serial queue order; the row stays
-    on the reference's CPU template (DESIGN.md section 0, f3)."""
-    import ctypes as C
+    on the reference's CPU template (DESIGN.md section 0, f3).  The reference's results are stored whole
+    (tests/golden/make_golden.py::epsilon_fill)."""
     import heapq
-    R = oracle.ref()
-    f = R.lib.ref_priority_flood_epsilon_f32
-    f.argtypes = [np.ctypeslib.ndpointer(np.float32, flags="C_CONTIGUOUS"), C.c_int, C.c_int, C.c_float]
-    f.restype = None
+    g = golden["epsilon_fill_ref"]
 
     def fixed_point(z):  # Dijkstra on the cost max(Z(c), nextafter(cost of the predecessor))
         h, w = z.shape
@@ -254,12 +263,13 @@ def test_epsilon_fill_depends_on_the_queue_order():
     above, cells = 0, 0
     for seed in (2, 5, 7):
         z = oracle.fbm_terrain(60, 80, seed=seed, quantum=0.5)
-        ref = z.copy()
-        f(ref, 80, 60, ND)
+        assert np.array_equal(z, g[f"s{seed}__dem"]), "terrain generator drifted"
+        ref = g[f"s{seed}__epsilon_filled"]
         fp = fixed_point(z)
         d = ref.view(np.int32).astype(np.int64) - fp.view(np.int32).astype(np.int64)
-        assert d.min() >= 0, "the serial result is never below the order-free fixed point"
-        assert d.max() <= 16
+        below = np.argwhere(d < 0)
+        assert not len(below), f"seed {seed}: the serial result is never below the order-free fixed point ({len(below)} cells, first {below[0]})"
+        assert d.max() <= 16, f"seed {seed}: {d.max()} ulps above the fixed point at {np.unravel_index(d.argmax(), d.shape)}"
         above += int((d > 0).sum())
         cells += z.size
         assert np.array_equal(ref >= z, np.ones_like(z, bool))
